@@ -2,14 +2,15 @@
 """Benchmark of the text->mel hot path (BASELINE.json configs[1]: LJSpeech ForwardTransformer 6+6 layers, d=256,
 inference, batch 64 per GPU, 128 phonemes -> 1000 mel frames, durations/pitch forced).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16x3|bf16]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16x3|bf16] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  `value` = mel frames/s with inputs resident in HBM, CUDA-event timed, max over
 ranks; `e2e` = the same metric through ForwardTransformer.predict() with host inputs (pinned H2D) and the mel copied
 back to the host every step; `roofline` = decoder conv GEMM launches (the dominant kernel) timed with CUDA events in
 the same run; `cpu_baseline` = the CPU oracle (torch fp32, all host cores) on a bounded sample of the same workload.
 `--impl reference` times only that CPU path (the reference is TF2 and cannot be installed offline; the oracle is its
-literal restatement).
+literal restatement).  `--dump-outputs DIR` writes what the last timed step returned (rank 0) as DIR/<name>.npy; inputs
+and weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -32,6 +33,7 @@ WORKLOAD = 'C2: LJ256 ForwardTransformer inference, B=64/GPU, 128 phonemes -> 10
 CFG_NAME = 'LJ256'
 B, TP, TM = 64, 128, 1000
 METRIC, UNIT = 'mel_frames_per_sec_fwd', 'frames/s'
+DUMP_LIMIT = 64 << 20
 
 
 def _traffic(key):
@@ -144,6 +146,26 @@ def _tf_reference_available() -> bool:
         return False
 
 
+def dump_outputs(dirname, out):
+    """The arrays of one step's result dict as DIR/<name>.npy (nested dicts as <name>.<key>.npy; None entries, such as
+    attention maps that were not requested, carry no array): floating-point arrays in float32, integer and boolean ones in
+    float64 (exact)."""
+    import numpy as np
+    arrays = {}
+    for k, v in out.items():
+        for sub, t in (v.items() if isinstance(v, dict) else [(None, v)]):
+            if t is None:
+                continue
+            a = t.detach().cpu()
+            arrays[k if sub is None else f'{k}.{sub}'] = (a.float() if a.is_floating_point() else a.double()).numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f'--dump-outputs: {total / 2**20:.0f} MB of outputs exceed the {DUMP_LIMIT >> 20} MB limit')
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + '.npy'), a)
+
+
 def _config_dict(world):
     return {'workload': WORKLOAD, 'model': CFG_NAME, 'global_batch': B * world, 'seq_len': TM}
 
@@ -172,8 +194,8 @@ def cpu_forward_rate(budget_s, min_passes=1, max_passes=8):
 
 def cpu_reference_line(args, rank, world):
     """--impl reference: the CPU path (oracle restatement of the TF2 graph) on the host cores.  Every step is the whole
-    64-row batch of the GPU arm's step (same config); when K+W whole steps do not fit the time budget the number of steps
-    actually run is reduced (and stated), never the step."""
+    64-row batch of the GPU arm's step (same config), and exactly --steps of them are timed; warm-up passes beyond the
+    first are capped at 15 % of a 240 s budget."""
     from oracle import forward_oracle as fo
     if rank != 0:
         return None
@@ -194,7 +216,7 @@ def cpu_reference_line(args, rank, world):
     t1 = time.perf_counter() - t0
     budget = 240.0
     warm = max(0, min(args.warmup - 1, int(0.15 * budget / t1)))
-    steps = max(1, min(args.steps, int((budget - (1 + warm) * t1) / t1)))
+    steps = args.steps
     for _ in range(warm):
         run()
     t0 = time.perf_counter()
@@ -202,7 +224,7 @@ def cpu_reference_line(args, rank, world):
         run()
     dt = time.perf_counter() - t0
     val = B * TM * steps / dt
-    sample = (f'{steps} whole steps of {B} rows x {TM} frames (asked for {args.steps}; a whole step takes {t1:.1f} s on this host), '
+    sample = (f'{steps} whole steps of {B} rows x {TM} frames (a whole step takes {t1:.1f} s on this host), '
               f'torch-CPU fp32 oracle, {cores} threads')
     return {'impl': 'reference', 'metric': METRIC, 'value': val, 'unit': UNIT, 'n_gpus': args.gpus, 'steps': steps,
             'warmup': warm + 1, 'ms_per_step': dt / steps * 1e3, 'higher_is_better': True, 'scaling': 'weak',
@@ -225,7 +247,7 @@ def hbm_bench(args, rank, world, dev, cfg):
     from transformertts_b200.data.audio import Audio
     _, peak_hbm, _ = _peaks()
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev)  # > 126 MB L2
-    steps = max(args.steps, 10)
+    steps = args.steps
     times = []
     if args.mode == 'stft':
         n_clips, n_samples = 256, 220500
@@ -545,7 +567,13 @@ def main():
     ap.add_argument('--mode', default='infer', choices=['infer', 'train', 'stft', 'expand', 'aligner'],
                     help="'train': BASELINE configs[2] (fwd+bwd+Adam, bf16, batch 32/GPU, NCCL data parallel); 'stft': configs[3] "
                          "(STFT->mel, 256 clips x 10 s); 'expand': the length regulator alone (C2-LR)")
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='default mode: write the outputs of the last timed step (rank 0) as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'ours' or args.mode != 'infer'):
+        ap.error('--dump-outputs applies to the default inference workload (--impl ours --mode infer)')
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
 
     rank = int(os.environ.get('RANK', '0'))
@@ -615,6 +643,8 @@ def main():
     barrier()
     launches = lib.launch_count()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

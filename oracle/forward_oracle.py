@@ -7,10 +7,10 @@ checker / reported CPU baseline.
 
 PARITY STATUS: the reference's arithmetic lives in TensorFlow/Keras (``tensorflow>=2.2.0``, ``requirements.txt:7``), which
 is not installed here and cannot be installed (no network), and the reference's own tests hold no golden vectors for this
-path (SURVEY.md section 4).  This restatement is pinned to the REFERENCE'S OWN CODE instead: tests/test_reference_shim.py
-imports the unmodified /root/reference/model/{layers,models,transformer_utils}.py and utils/losses.py, runs them on
+path (SURVEY.md section 4).  This restatement is pinned to the REFERENCE'S OWN CODE instead: tests/golden/make_reference_pins.py
+imports the unmodified model/{layers,models,transformer_utils}.py and utils/losses.py of the reference, runs them on
 tests/tf_shim (a torch-backed stand-in for the TensorFlow/Keras primitives, semantics from the TF documentation; the
-reference's tests/test_loss.py known answers pass on it) and compares ``ForwardTransformer.call`` / ``predict`` / ``_train_step``
+reference's tests/test_loss.py known answers pass on it), and tests/test_reference_shim.py compares ``ForwardTransformer.call`` / ``predict`` / ``_train_step``
 (loss, every gradient, Keras Adam) with this file on C1 / LJ256 / LJ256-dense / REF384: agreement 2e-5 (mel), 1e-5 (attention),
 bit-exact masks and integer durations.  The golden vectors tests/golden/{c1_forward,ref_lj256,ref_train_c1}.npz are written by
 those reference-code runs (tests/golden/make_golden_ref.py; make_golden_tf.py does the same on a machine with real TensorFlow).

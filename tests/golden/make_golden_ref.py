@@ -1,8 +1,8 @@
-"""Golden vectors produced by the REFERENCE'S OWN CODE (run in the build container, where /root/reference exists):
+"""Golden vectors produced by the REFERENCE'S OWN CODE:
 
-    python tests/golden/make_golden_ref.py
+    TTS_REFERENCE=<checkout of as-ideas/TransformerTTS> python tests/golden/make_golden_ref.py
 
-The unmodified /root/reference/model/models.py (ForwardTransformer, Aligner) is imported and executed on top of
+The unmodified model/models.py of the reference (ForwardTransformer, Aligner) is imported and executed on top of
 tests/tf_shim -- a torch-backed stand-in for the TensorFlow/Keras primitives, because TensorFlow cannot be installed in
 this image (see tests/tf_shim/README.md; tests/golden/make_golden_tf.py is the same script for a machine that has the real
 TensorFlow).  Weights are the seed-7 set of oracle.forward_oracle.init_params mapped onto the Keras variables; inputs come

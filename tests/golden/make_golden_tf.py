@@ -1,6 +1,6 @@
 """Golden vectors from the UNMODIFIED reference on REAL TensorFlow (SURVEY.md 8c: "prefer the real reference if it appears").
 
-    python tests/golden/make_golden_tf.py        # needs `import tensorflow` (>= 2.2) and /root/reference (or $TTS_REFERENCE)
+    python tests/golden/make_golden_tf.py        # needs `import tensorflow` (>= 2.2) and $TTS_REFERENCE
 
 This image has no TensorFlow wheel and no network, so this script cannot run here; it is committed so that anyone with a
 TensorFlow box can regenerate tests/golden/*.npz from the real thing and re-run the suite.  It is the same program as

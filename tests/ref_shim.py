@@ -1,20 +1,20 @@
-"""Helpers that run the UNMODIFIED reference sources (/root/reference) on top of tests/tf_shim (test infrastructure only).
-
-`available()` is False where /root/reference does not exist (the GPU box): the tests that need it skip there and use the
-golden vectors this module's users committed under tests/golden/ instead."""
+"""Helpers that run the UNMODIFIED reference sources on top of tests/tf_shim, for the scripts under tests/golden/ that
+write the golden vectors.  The reference is a checkout of as-ideas/TransformerTTS named by the TTS_REFERENCE environment
+variable; the tests themselves only read the committed golden files."""
 from __future__ import annotations
 
+import os
 import sys
 from pathlib import Path
 
 import torch
 
-REFERENCE = Path('/root/reference')
+REFERENCE = Path(os.environ['TTS_REFERENCE']) if os.environ.get('TTS_REFERENCE') else None
 SHIM = Path(__file__).resolve().parent / 'tf_shim'
 
 
 def available() -> bool:
-    return (REFERENCE / 'model' / 'models.py').exists()
+    return REFERENCE is not None and (REFERENCE / 'model' / 'models.py').exists()
 
 
 def real_tensorflow_available() -> bool:
@@ -27,7 +27,7 @@ def real_tensorflow_available() -> bool:
 def activate(real_tf: bool = False):
     """Put the reference tree (and, unless real_tf, the shim packages) on sys.path (idempotent)."""
     if not available():
-        raise RuntimeError('/root/reference is not present on this machine')
+        raise RuntimeError('set TTS_REFERENCE to a checkout of as-ideas/TransformerTTS')
     paths = (str(REFERENCE),) if real_tf else (str(REFERENCE), str(SHIM))
     for p in paths:
         if p in sys.path:
@@ -122,7 +122,7 @@ def aligner_named_parameters(model, cfg: dict) -> dict:
 
 
 def reference_forward_transformer(cfg: dict, params: dict, warm_inputs, **overrides):
-    """Instantiate /root/reference/model/models.py:ForwardTransformer (unmodified) under the shim with `params`.
+    """Instantiate the reference's model/models.py:ForwardTransformer (unmodified) under the shim with `params`.
     `warm_inputs` = (tokens, durations (B,Tp,1), pitch (B,Tp,1)): one throw-away call creates the Keras variables (the
     reference's own build_model_weights() feeds a 1x1 dummy, which produces an empty decoder input)."""
     activate()
@@ -143,7 +143,7 @@ def reference_forward_transformer(cfg: dict, params: dict, warm_inputs, **overri
 
 
 def reference_aligner(cfg: dict, params: dict, warm_inputs, **overrides):
-    """Instantiate /root/reference/model/models.py:Aligner (unmodified) under the shim with `params`."""
+    """Instantiate the reference's model/models.py:Aligner (unmodified) under the shim with `params`."""
     activate()
     from model.models import Aligner  # the reference class
     kw = {k: v for k, v in cfg.items() if k not in ('vocab_size', 'stop_loss_scaling')}

@@ -1,7 +1,7 @@
 """Test-only TensorFlow shim on torch CPU tensors (see tests/tf_shim/README.md).
 
 Implements exactly the TF 2.x / Keras entry points the reference's text->mel path uses, with the semantics of the TF
-documentation, so that the UNMODIFIED files under /root/reference can be imported and executed.  Tensors are plain
+documentation, so that the UNMODIFIED files of the reference can be imported and executed.  Tensors are plain
 ``torch.Tensor``; ``tf.Variable`` is a ``torch.nn.Parameter`` subclass; ``tf.GradientTape`` is torch autograd.
 
 Known deviations (none on the ForwardTransformer path): ``int / int`` is float32 true division here, float64 in TF
