@@ -129,7 +129,8 @@ typedef struct ttsb_gemm_args {
   int out_fp16;             /* 1: out_hi receives IEEE fp16 (single plane) instead of bf16 hi/lo */
   float* out_preln;         /* optional fp32 (B,T,ld_out): value before the LayerNorm (saved for the backward pass) */
   /* training dropout (keras semantics, stateless mask from (seed, site, element index)): drop_pre on the GEMM output
-   * after bias/ReLU and before the residual add; drop_post on the LayerNorm output */
+   * after bias/ReLU and before the residual add; drop_post on the LayerNorm output.  The element index of output column
+   * n of row (b, t) is (b*T + t)*ld_out + n for both sites (the offset of the element in out_f32 / out_preln). */
   float drop_pre_p, drop_post_p;
   uint32_t drop_pre_site, drop_post_site, drop_seed;
   int precision;            /* TTSB_PREC_* */
@@ -261,7 +262,8 @@ int ttsb_wgrad(const ttsb_wgrad_args* args, void* stream);
 int ttsb_rowdot_heads(const void* x_bf16, const void* y_bf16, int B, int T, int H, int dh, int ld, float* out, void* stream);
 
 /* Row softmax of materialised, pre-scaled scores S fp32 (B*H, T, ld) with key masking (model/layers.py:186-192) and
- * attention dropout: P_pre = softmax, P_drop = dropout(P_pre) (pass the same pointer twice when drop_p == 0). */
+ * attention dropout: P_pre = softmax, P_drop = dropout(P_pre) (pass the same pointer twice when drop_p == 0).  Dropout
+ * element index of key k in row t of problem z = b*H + h: (z*T + t)*ld + k (ttsb_softmax_bwd regenerates the same mask). */
 /* flags: bit 0 = look-ahead mask (keys > query index masked, transformer_utils.py:35-37); bit 1 = every query row is live
  * (Aligner blocks); without it query rows >= kv_len[b] are written as zeros (they are masked downstream). */
 int ttsb_softmax_fwd(const float* S, int B, int H, int T, int Tk, int ld, const int32_t* kv_len, float drop_p,
@@ -285,7 +287,10 @@ int ttsb_attn_ds_bwd(const void* dO, int ld_do, int do_col0, const void* v, int 
                      uint32_t site, void* dS, int ld_p, void* stream);
 int ttsb_softmax_bwd(const void* P_pre, const float* dP, int B, int H, int T, int Tk, int ld, const int32_t* kv_len,
                      float scale, float drop_p, uint32_t seed, uint32_t site, int flags, void* dS, void* stream);
-/* LayerNorm backward from the saved pre-norm values u (keras LayerNormalization, model/layers.py:27,96,207,295,508). */
+/* LayerNorm backward from the saved pre-norm values u (keras LayerNormalization, model/layers.py:27,96,207,295,508).
+ * post_drop regenerates the mask of a dropout on the LayerNorm output (applied to dz), pre_drop that of ttsb_linear_fwd's
+ * drop_pre (applied to g_bf16, the gradient of the GEMM output); both use element index (b*T + t)*ld + c, the index
+ * ttsb_linear_fwd uses with ld_out = ld. */
 int ttsb_layernorm_bwd(const float* dz, const float* u, const float* gamma, int B, int T, int C, int ld, float eps,
                        const int32_t* row_len, int relu_mask, float pre_drop_p, uint32_t pre_site, float post_drop_p,
                        uint32_t post_site, uint32_t seed, float* du, void* g_bf16, float* dgamma, float* dbeta, float* dbias,
@@ -331,12 +336,17 @@ int ttsb_diag_loss_train(const void* P_bf16, int B, int H, int Tq, int Tk, int l
                          float loss_scale, float* loss_out, float grad_scale, float* dP, void* stream);
 int ttsb_diag_loss(const float* att, int B, int H, int Tq, int Tk, const int32_t* q_len, const int32_t* k_len,
                    float* loss_out, void* stream);
+/* Expand (length regulator) backward: dx[b,i,:] = sum of dm[b,t,:] over the frames t in [start_i, start_i + dur[b,i]) with
+ * start_i = sum_{j<i} max(dur[b,j], 0); negative durations count as 0 and frames >= Tm are dropped.  dm fp32 (B,Tm,d), dx fp32
+ * (B,Tp,d) (every element written); d must be a multiple of 4 and dm, dx 16-byte aligned (float4 rows). */
 int ttsb_expand_bwd(const float* dm, const int32_t* dur_int, int B, int Tp, int Tm, int d, float* dx, void* stream);
 int ttsb_embedding_bwd(const float* dx, const int32_t* tokens, int B, int T, int d, int vocab, float* demb, void* stream);
-/* d(pos_encoding_scalar) = sum dropout(g) * PE[t]; (drop_p, seed, site) regenerate the prologue dropout mask */
+/* d(pos_encoding_scalar) = sum dropout(g) * PE[t]; (drop_p, seed, site) regenerate the prologue dropout mask (element index
+ * (b*T + t)*d + c, the flat index of the prologue output) */
 int ttsb_pe_scalar_bwd(const float* g, const float* pe, int B, int T, int d, float drop_p, uint32_t seed, uint32_t site,
                        float* dscalar, void* stream);
-/* training variants of the two stack prologues: keras Dropout after LayerNorm + PE (model/layers.py:301) */
+/* training variants of the two stack prologues: keras Dropout after LayerNorm + PE (model/layers.py:301); dropout element
+ * index = flat output index (b*T + t)*d + c (T = Tm for the expand form) */
 int ttsb_embed_ln_pe_train_fwd(const int32_t* tokens, const float* emb, const float* gamma, const float* beta,
                                const float* pe, const float* pos_scalar, int B, int T, int d, int vocab, float eps,
                                float drop_p, uint32_t seed, uint32_t site, float* out_f32, void* out_hi, void* out_lo,

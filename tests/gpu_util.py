@@ -1,6 +1,7 @@
 """Helpers shared by the GPU parity tests: drive single kernels of libttsb.so through the C ABI."""
 from __future__ import annotations
 
+import numpy as np
 import torch
 
 from transformertts_b200 import lib
@@ -13,9 +14,31 @@ def split_or_none(x: torch.Tensor, split: bool):
     return lib.split_bf16(x, split)
 
 
+def dropout_keep_host(idx, p, seed, site, salt=0):
+    """Host restatement of the library's stateless dropout mask (csrc/ttsb_common.cuh: dropout_keep): True where element
+    `idx` (any integer array) of dropout site `site` is kept at rate p (float32, as the kernels receive it)."""
+    idx = np.asarray(idx, dtype=np.uint64)
+    pair = idx >> np.uint64(1)
+    u32 = lambda v: np.uint32(int(v) & 0xffffffff)
+    hterm = ((pair >> np.uint64(32)).astype(np.uint32) * u32(0x85EBCA77)) ^ u32(((seed ^ salt) & 0xffffffff) * 0xC2B2AE3D) \
+        ^ u32(site * 0x27D4EB2F)
+    x = (pair & np.uint64(0xffffffff)).astype(np.uint32) * u32(0x9E3779B1) ^ hterm
+    x ^= x >> np.uint32(16)
+    x *= u32(0x7FEB352D)
+    x ^= x >> np.uint32(15)
+    x *= u32(0x846CA68B)
+    x ^= x >> np.uint32(16)
+    half = np.where((idx & np.uint64(1)) != 0, x >> np.uint32(16), x & np.uint32(0xffff))
+    thresh = int(float(np.float32(p)) * 4294967296.0) if p > 0 else 0
+    return half >= np.uint32(thresh >> 16)
+
+
 def run_gemm(x_list, w_kn, bias, seg_src, seg_shift, seg_k, *, precision='bf16x3', impl='tcgen05', relu=False,
-             residual=None, ln=None, row_len=None, block_n=None, single_tile=False, out_fp16=False):
-    """x_list: fp32 (B,T,C) sources (on GPU).  Returns dict with requested outputs."""
+             residual=None, ln=None, row_len=None, block_n=None, single_tile=False, out_fp16=False, drop_pre=None,
+             drop_post=None, drop_seed=0, out_preln=False, want_f32=True):
+    """x_list: fp32 (B,T,C) sources (on GPU).  Returns dict with requested outputs.  drop_pre / drop_post: (rate, site) of
+    the two dropout sites of the epilogue; out_preln=True also returns the saved pre-LayerNorm values ('preln');
+    want_f32=False leaves out_f32 NULL (16-bit outputs only).  'launches' counts the kernels ttsb_linear_fwd launched."""
     split = precision == 'bf16x3'
     B, T, _ = x_list[0].shape
     pl = _PackedLinear(w_kn, bias, seg_k, split, single_tile=single_tile, block_n=block_n)
@@ -51,24 +74,38 @@ def run_gemm(x_list, w_kn, bias, seg_src, seg_shift, seg_k, *, precision='bf16x3
     out_f32 = torch.full((B, T, pl.n_pad), float('nan'), device=DEV)
     out_hi = torch.full((B, T, pl.n_pad), float('nan'), device=DEV, dtype=torch.bfloat16)
     out_lo = torch.full((B, T, pl.n_pad), float('nan'), device=DEV, dtype=torch.bfloat16)
-    a.out_f32, a.out_hi = out_f32.data_ptr(), out_hi.data_ptr()
+    a.out_f32, a.out_hi = (out_f32.data_ptr() if want_f32 else None), out_hi.data_ptr()
     a.out_lo = out_lo.data_ptr() if split else None
     a.ld_out = pl.n_pad
     a.out_fp16 = int(out_fp16)
+    preln = None
+    if out_preln:
+        preln = torch.full((B, T, pl.n_pad), float('nan'), device=DEV)
+        a.out_preln = preln.data_ptr()
+    if drop_pre is not None:
+        a.drop_pre_p, a.drop_pre_site = drop_pre
+    if drop_post is not None:
+        a.drop_post_p, a.drop_post_site = drop_post
+    a.drop_seed = drop_seed
     a.precision = lib.PREC_BF16X3 if split else lib.PREC_BF16
     a.impl = lib.IMPL_SIMT if impl == 'simt' else lib.IMPL_TCGEN05
+    n0 = lib.launch_count()
     lib.linear_fwd(a)
+    out['launches'] = lib.launch_count() - n0
     torch.cuda.synchronize()
-    out['f32'] = out_f32
+    out['f32'] = out_f32 if want_f32 else None
     out['hi'] = out_hi
     out['lo'] = out_lo if split else None
     out['n_pad'] = pl.n_pad
+    out['preln'] = preln
     return out
 
 
-def ref_gemm(x_list, w_kn, bias, seg_src, seg_shift, seg_k, *, precision, relu=False, residual=None, ln=None, row_len=None):
+def ref_gemm(x_list, w_kn, bias, seg_src, seg_shift, seg_k, *, precision, relu=False, residual=None, ln=None, row_len=None,
+             drop_pre=None, drop_post=None, drop_seed=0, salt=0, ld_out=None, return_preln=False):
     """float64 CPU reference of the same contract.  In 'bf16' mode the operands are first rounded to bf16 (that is the
-    kernel's arithmetic); in 'bf16x3' mode the fp32 operands are used as they are."""
+    kernel's arithmetic); in 'bf16x3' mode the fp32 operands are used as they are.  Dropout uses the host mask at element
+    index (b*T + t)*ld_out + n; return_preln=True returns (output, pre-LayerNorm value)."""
     xs = [x.detach().cpu().double() if precision == 'bf16x3' else x.detach().cpu().bfloat16().double() for x in x_list]
     w = w_kn.detach().cpu().reshape(-1, w_kn.shape[-1])
     w = w.double() if precision == 'bf16x3' else w.bfloat16().double()
@@ -87,17 +124,29 @@ def ref_gemm(x_list, w_kn, bias, seg_src, seg_shift, seg_k, *, precision, relu=F
         acc += bias.detach().cpu().double()
     if relu:
         acc = torch.relu(acc)
+
+    def drop(v, rate_site):
+        rate, site = rate_site
+        idx = (np.arange(B * T, dtype=np.uint64)[:, None] * np.uint64(ld_out) + np.arange(N, dtype=np.uint64)[None, :])
+        keep = torch.from_numpy(dropout_keep_host(idx, rate, drop_seed, site, salt)).view(B, T, N)
+        return v * keep / (1.0 - float(np.float32(rate)))
+
+    if drop_pre is not None and drop_pre[0] > 0:
+        acc = drop(acc, drop_pre)
     if residual is not None:
         acc += residual.detach().cpu().double()[..., :N]
+    preln = acc.clone()
     if ln is not None:
         g, b = ln[0].detach().cpu().double(), ln[1].detach().cpu().double()
         mean = acc.mean(-1, keepdim=True)
         var = ((acc - mean) ** 2).mean(-1, keepdim=True)
         acc = (acc - mean) * torch.rsqrt(var + 1e-6) * g + b
+    if drop_post is not None and drop_post[0] > 0:
+        acc = drop(acc, drop_post)
     if row_len is not None:
         keep = torch.arange(T)[None, :] < row_len.detach().cpu()[:, None]
         acc = acc * keep[..., None]
-    return acc
+    return (acc, preln) if return_preln else acc
 
 
 def _to16(x, precision, split):

@@ -71,6 +71,12 @@ def test_argument_validation_without_gpu(cdll):
     assert b'ttsb_attn_probs_fwd' in cdll.ttsb_last_error()
     assert cdll.ttsb_attn_ds_bwd(None, 256, 0, None, 768, 512, 1, 2, 100, 128, None, None, None, C.c_float(0.1), C.c_float(0.1), 0, 0, None, 112, None) == -1
     assert b'ttsb_attn_ds_bwd' in cdll.ttsb_last_error()
+    # Expand backward walks rows as float4: d % 4 != 0 and unaligned rows are refused (the pointers are never dereferenced)
+    dur = C.c_void_p(0x1000)
+    assert cdll.ttsb_expand_bwd(C.c_void_p(0x2000), dur, 1, 4, 8, 6, C.c_void_p(0x3000), None) == -1
+    assert b'ttsb_expand_bwd' in cdll.ttsb_last_error()
+    assert cdll.ttsb_expand_bwd(C.c_void_p(0x2004), dur, 1, 4, 8, 128, C.c_void_p(0x3000), None) == -1
+    assert cdll.ttsb_expand_bwd(C.c_void_p(0x2000), dur, 1, 4, 8, 128, C.c_void_p(0x3008), None) == -1
 
 
 def test_product_package_never_imports_the_oracle():

@@ -729,11 +729,6 @@ __global__ void expand_bwd_kernel(const float* __restrict__ dm, const int* __res
       }
       reinterpret_cast<float4*>(dx + ((size_t)b * Tp + i) * d)[c] = make_float4(a0.x + a1.x, a0.y + a1.y, a0.z + a1.z, a0.w + a1.w);
     }
-    for (int c = (d4 << 2) + lane; c < d; c += 32) {   // d % 4 tail
-      float acc = 0.f;
-      for (int t = s; t < e; ++t) acc += dm[((size_t)b * Tm + t) * d + c];
-      dx[((size_t)b * Tp + i) * d + c] = acc;
-    }
   }
 }
 
@@ -1018,6 +1013,9 @@ extern "C" int ttsb_rowdot_heads(const void* x, const void* y, int B, int T, int
 
 extern "C" int ttsb_expand_bwd(const float* dm, const int32_t* dur_int, int B, int Tp, int Tm, int d, float* dx, void* stream) {
   if (!dm || !dur_int || !dx || B <= 0 || Tp <= 0 || Tm <= 0 || d <= 0) return bad("ttsb_expand_bwd: bad arguments");
+  // the kernel walks rows as float4 columns: dm / dx rows start 16-byte aligned only when d % 4 == 0
+  if (d % 4 || (reinterpret_cast<uintptr_t>(dm) & 15) || (reinterpret_cast<uintptr_t>(dx) & 15))
+    return bad("ttsb_expand_bwd: d must be a multiple of 4 and dm, dx 16-byte aligned");
   const int chunks = std::min(32, (Tp + 7) / 8);
   expand_bwd_kernel<<<dim3(B, chunks), 256, (Tp + 1) * sizeof(int), STREAM(stream)>>>(dm, dur_int, Tp, Tm, d, dx);
   LAUNCH_OK("expand_bwd_kernel");
